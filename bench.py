@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--config K16|N4|R8|T1|LPG]    # our arm (torchrun launches N>1)
     python bench.py --impl reference --gpus N --steps K ...                      # reference arm: the reference on host cores
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step computed to DIR/<name>.npy
 
 Default workload K16 (BASELINE.json configs[1], the config the metric is quoted on): DenseNet-161 encoder, 352x704
 synthetic RGB->depth, batch 16 PER GPU (weak scaling), train mode (batch-stat BN), silog loss (lambda .85), backward,
@@ -198,8 +199,9 @@ def _reference_model(cfg, torch):
     return m, (lambda est, gt, mask: O.silog(est, gt, mask, 0.85)), "port", "oracle/bts_oracle.py OracleModel"
 
 
-def cpu_reference_steps(cfg, steps, warmup, B=2, budget_s=150.0):
-    """The reference on all host cores: one train step (or eval forward for T1) per sample batch of B images."""
+def cpu_reference_steps(cfg, steps, warmup, B=2, budget_s=None):
+    """The reference on all host cores: one train step (or eval forward for T1) per sample batch of B images.
+    budget_s: stop timing after this many seconds (bounded sample), else run every step."""
     import torch
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import ref_shim
@@ -216,7 +218,7 @@ def cpu_reference_steps(cfg, steps, warmup, B=2, budget_s=150.0):
         times = []
         t_start = time.perf_counter()
         for i in range(warmup + steps):
-            if times and time.perf_counter() - t_start > budget_s:
+            if budget_s is not None and times and time.perf_counter() - t_start > budget_s:
                 break                                  # bounded sample: keep the bench within minutes on slow hosts
             t0 = time.perf_counter()
             if train:
@@ -426,14 +428,14 @@ def run_lpg_config(args):
     for r in (8, 4, 2):
         for side in (256, 384, 512, 768, 1024):
             Bh = max(16, (512 * 1024 * 1024 + 4 * side * side - 1) // (4 * side * side))
-            a = _lpg_time(torch, dev, Bh, side, r)
-            b = _lpg_time(torch, dev, 16, side, r, reps=10, flush=flush)
+            a = _lpg_time(torch, dev, Bh, side, r, reps=args.steps)
+            b = _lpg_time(torch, dev, 16, side, r, reps=args.steps, flush=flush)
             rows.append({"r": r, "side": side, "hbm": {k: a[k] for k in ("B", "fwd_ms", "bwd_ms", "fwd_gbs", "bwd_gbs", "fwd_bwd_gbs")},
                          "b16": {k: b[k] for k in ("B", "fwd_ms", "bwd_ms", "fwd_gbs", "bwd_gbs", "fwd_bwd_gbs")}})
             torch.cuda.empty_cache()
     vals = [x["hbm"]["fwd_bwd_gbs"] for x in rows]
     res = {"metric": "LPG fwd+bwd GB/s vs HBM peak", "value": statistics.median(vals), "unit": "GB/s", "n_gpus": 1,
-           "steps": 20, "warmup": 3, "ms_per_step": None, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+           "steps": args.steps, "warmup": 3, "ms_per_step": None, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
            "dtype": "f32", "data": "synthetic",
            "config": {"workload": "LPG-u: plane-to-depth fwd+bwd, r=8/4/2, H=W 256..1024, 1 GPU; value = median over the 15 "
                                   "HBM-regime points", "l2": "hbm regime: outputs >= 512 MB; b16 regime: 256 MB flush write between launches"},
@@ -642,6 +644,31 @@ def conv_rooflines(torch, conv, step_fn, pk_tf32):
     return out
 
 
+OUTPUT_NAMES = ("depth_8x8_scaled", "depth_4x4_scaled", "depth_2x2_scaled", "reduc1x1", "final_depth")
+DUMP_CAP = 1 << 21        # elements per dumped array: at most 7 arrays of 8 MiB (float32), under 64 MiB in all
+
+
+def dump_outputs(path, keep, model, train, torch):
+    """--dump-outputs: what the last timed step computed, as <path>/<name>.npy in float32 -- the model's five outputs and,
+    for a training step, the loss, the parameters after the optimizer step and their gradients (each flattened in
+    model.parameters() order, frozen parameters have no gradient).  An array of more than DUMP_CAP elements is replaced
+    by the same fixed sample every run: the elements at the sorted first DUMP_CAP indices of a seed-0 permutation."""
+    import numpy as np
+    arrays = dict(zip(OUTPUT_NAMES, keep["out"]))
+    if train:
+        arrays["loss"] = keep["loss"]
+        ps = list(model.parameters())
+        arrays["params"] = torch.cat([q.detach().reshape(-1) for q in ps])
+        arrays["grads"] = torch.cat([q.grad.reshape(-1) for q in ps if q.grad is not None])
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_CAP:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_CAP].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def _run_ours(args):
     import torch
     import torch.distributed as dist
@@ -720,13 +747,20 @@ def _run_ours(args):
     himg, hfocal, hgt = synth_batch(cfg, B, 1 + rank, pin=True)
     total_steps = 10000
 
+    keep = {} if args.dump_outputs else None     # the last step's outputs and loss, for --dump-outputs
+
+    def graph_loss(out, g):
+        if keep is not None:
+            keep["out"] = out                    # the capture calls this last: these are the graph's static outputs
+        return crit(out[4], g, g > cfg["thr"])
+
     graphed = None
     graph_note = "off"
     if train and args.graph != "off" and args.reducer != "ddp":
         # forward + loss + backward of one step as ONE CUDA graph (bts_b200/graph.py); collective + optimizer stay eager
         try:
             from bts_b200.graph import GraphedTrainStep
-            graphed = GraphedTrainStep(model, lambda out, g: crit(out[4], g, g > cfg["thr"]), ((img, focal), (gt,)))
+            graphed = GraphedTrainStep(model, graph_loss, ((img, focal), (gt,)))
             graph_note = "fwd+loss+bwd captured in one CUDA graph (%d native launches per replay)" % graphed.launches_per_replay
         except Exception as e:
             if args.graph == "on":
@@ -740,7 +774,10 @@ def _run_ours(args):
     def step(i, x, f, g):
         if not train:
             with torch.no_grad():
-                return model(x, f)[4].sum()
+                out = model(x, f)
+            if keep is not None:
+                keep["out"] = out
+            return out[4].sum()
         if bcast is not None:
             bcast.broadcast(0)
         if graphed is not None:
@@ -750,6 +787,10 @@ def _run_ours(args):
             out = model(x, f)
             loss = crit(out[4], g, g > cfg["thr"])
             loss.backward()
+            if keep is not None:
+                keep["out"] = out
+        if keep is not None:
+            keep["loss"] = loss
         if red is not None:
             red.reduce(inplace=graphed is not None)
         lr = (1e-4 - 1e-5) * (1 - i / total_steps) ** 0.9 + 1e-5
@@ -812,6 +853,8 @@ def _run_ours(args):
         return float(step(i, x, f, g).detach())  # D2H read of the loss (bts_main.py:463) / of the result every step
 
     ms_e, _, _, per_e = timed(e2e_step, K, 1)
+    if keep is not None and rank == 0:
+        dump_outputs(args.dump_outputs, keep, model, train, torch)
     h2d = himg.numel() * 4 + hfocal.numel() * 8 + hgt.numel() * 4
 
     pk = peaks()
@@ -889,7 +932,7 @@ def _run_ours(args):
                 except Exception as e:
                     res["gpu_baseline"] = {"error": "%s: %s" % (type(e).__name__, e)}
             if not args.no_cpu:
-                res["cpu_baseline"] = cpu_reference_steps(cfg, 3, 1)
+                res["cpu_baseline"] = cpu_reference_steps(cfg, 3, 1, budget_s=150.0)
     return res, rank, (dist if world > 1 else None)
 
 
@@ -913,7 +956,7 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (launches per point for --config LPG)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="K16", choices=sorted(CONFIGS) + ["LPG"])
@@ -929,7 +972,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip the torch-eager/cuDNN reference leg")
     ap.add_argument("--no-roofline", action="store_true", help="skip every evidence leg (peaks, traced step, LPG, baselines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == "LPG"):
+        ap.error("--dump-outputs writes the outputs of our model's step: not with --impl reference or --config LPG")
     if args.selfcheck_child is not None:
         selfcheck_child(set(args.selfcheck_child.split(",")))
         return

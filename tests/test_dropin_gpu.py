@@ -7,7 +7,8 @@
   2. bts_test.py re-imports the model file by name from the checkpoint directory, loads that checkpoint into a
      DataParallel-wrapped BtsModel, runs inference and writes the 16-bit depth PNGs.
 
-The scripts come from oracle/_ref/ (copied there, unmodified, by `make -C oracle`; git-ignored) or /root/reference.
+The scripts are the reference's own source, so they are never committed: `make -C oracle` copies them, unmodified, from a
+checkout of the reference into the git-ignored oracle/_ref/, and the test skips where that copy is absent.
 tests/dropin/boot.py supplies the environment the 2019 scripts assume (stub tensorboardX / matplotlib, two torch-2.x
 compatibility shims) -- see its docstring."""
 import os
@@ -27,10 +28,8 @@ SCRIPTS = ["bts_main.py", "bts_test.py", "bts_dataloader.py", "distributed_sampl
 
 
 def _script_dir():
-    for d in ("/root/reference/pytorch", os.path.join(ROOT, "oracle", "_ref")):
-        if all(os.path.isfile(os.path.join(d, s)) for s in SCRIPTS):
-            return d
-    return None
+    d = os.path.join(ROOT, "oracle", "_ref")
+    return d if all(os.path.isfile(os.path.join(d, s)) for s in SCRIPTS) else None
 
 
 def _make_dataset(d, n=4):
@@ -51,7 +50,7 @@ def _make_dataset(d, n=4):
         f.write("\n".join(lines) + "\n")
 
 
-@pytest.mark.skipif(_script_dir() is None, reason="reference scripts not available (run `make -C oracle` where /root/reference exists)")
+@pytest.mark.skipif(_script_dir() is None, reason="reference scripts not in oracle/_ref (`make -C oracle REF=<reference>/pytorch`)")
 def test_unmodified_bts_main_and_bts_test_run_against_our_module(tmp_path):
     src = _script_dir()
     work = tmp_path / "work"

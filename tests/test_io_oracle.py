@@ -1,67 +1,38 @@
-"""CPU: pins oracle/io_oracle.py (the checker of csrc/io.cu) against the reference's own functions, executed live from the
-unmodified source where it is available (/root/reference or oracle/_ref): DataLoadPreprocess.augment_image /
-train_preprocess / ToTensor (pytorch/bts_dataloader.py) and compute_errors (pytorch/bts_main.py:144-165, extracted by
-ast because the script parses argv at import)."""
-import ast
-import os
+"""CPU: pins oracle/io_oracle.py (the checker of csrc/io.cu) against the reference's own functions, through their outputs
+stored in tests/golden/io_reference.npz (oracle/make_golden.py runs the unmodified source): DataLoadPreprocess.random_crop /
+train_preprocess / augment_image / ToTensor (pytorch/bts_dataloader.py) and compute_errors (pytorch/bts_main.py:144-165)."""
 import random
-import sys
-import types
 
 import numpy as np
 import pytest
 
 import io_oracle as IO
-from conftest import ROOT
 
 
-def _ref_dir():
-    for d in ("/root/reference/pytorch", os.path.join(ROOT, "oracle", "_ref")):
-        if os.path.isfile(os.path.join(d, "bts_dataloader.py")) and os.path.isfile(os.path.join(d, "bts_main.py")):
-            return d
-    return None
-
-
-needs_ref = pytest.mark.skipif(_ref_dir() is None, reason="reference sources not available")
-
-
-@needs_ref
-def test_compute_errors_matches_reference_function():
-    src = open(os.path.join(_ref_dir(), "bts_main.py")).read()
-    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "compute_errors"][0]
-    ns = {"np": np}
-    exec(compile(ast.Module([fn], []), "bts_main.compute_errors", "exec"), ns)
+def test_compute_errors_matches_reference_function(golden):
+    want = golden("io_reference")["compute_errors"]
     rng = np.random.RandomState(0)
     gt = rng.uniform(0.5, 70, 5000).astype(np.float32)
     pred = (gt * rng.uniform(0.6, 1.6, 5000)).astype(np.float32)
-    want = ns["compute_errors"](gt, pred)
     got = IO.compute_errors(gt, pred)
-    np.testing.assert_allclose(np.array(got, dtype=np.float64), np.array(want, dtype=np.float64), rtol=1e-6)
+    np.testing.assert_allclose(np.array(got, dtype=np.float64), want, rtol=1e-6)
 
 
-@needs_ref
 @pytest.mark.parametrize("dataset", ["nyu", "kitti"])
-def test_input_prep_matches_reference_loader_transform(dataset):
-    sys.path.insert(0, _ref_dir())
-    import importlib
-    D = importlib.import_module("bts_dataloader")
-    args = types.SimpleNamespace(dataset=dataset)
-    ds = D.DataLoadPreprocess.__new__(D.DataLoadPreprocess)
-    ds.args = args
+def test_input_prep_matches_reference_loader_transform(golden, dataset):
+    g = golden("io_reference")
     rng = np.random.RandomState(1)
     img_u8 = rng.randint(0, 256, (40, 56, 3)).astype(np.uint8)
     dep_u16 = rng.randint(0, 60000, (40, 56)).astype(np.uint16)
     div = 1000.0 if dataset == "nyu" else 256.0
     H, W = 32, 32
+    assert len(g[dataset + "_image"]) == 6
     for seed in range(6):
         # replay the reference's own random draws: random_crop (x then y), flip, do_augment, gamma, brightness, np colours
         random.seed(seed)
         np.random.seed(seed)
-        image = np.asarray(img_u8, dtype=np.float32) / 255.0
-        depth = np.expand_dims(np.asarray(dep_u16, dtype=np.float32), 2) / div
-        st = random.getstate()
-        x0 = random.randint(0, image.shape[1] - W)
-        y0 = random.randint(0, image.shape[0] - H)
+        x0 = random.randint(0, img_u8.shape[1] - W)
+        y0 = random.randint(0, img_u8.shape[0] - H)
         do_flip = random.random()
         do_aug = random.random()
         gamma = brightness = 1.0
@@ -70,12 +41,7 @@ def test_input_prep_matches_reference_loader_transform(dataset):
             gamma = random.uniform(0.9, 1.1)
             brightness = random.uniform(0.75, 1.25) if dataset == "nyu" else random.uniform(0.9, 1.1)
             colors = np.random.uniform(0.9, 1.1, size=3)
-        random.setstate(st)
-        np.random.seed(seed)
-        ci, cd = ds.random_crop(image, depth, H, W)
-        ri, rd = ds.train_preprocess(ci, cd)
-        sample = D.ToTensor("train")({"image": ri, "depth": rd, "focal": 1.0})
-        want_i, want_d = sample["image"].numpy(), sample["depth"].numpy()
+        want_i, want_d = g[dataset + "_image"][seed], g[dataset + "_depth"][seed]
         got_i, got_d = IO.input_prep(img_u8, dep_u16, div, y0, x0, H, W, do_flip > 0.5, do_aug > 0.5, gamma, brightness, colors)
         np.testing.assert_allclose(got_i, want_i, rtol=1e-6, atol=1e-6)
         np.testing.assert_array_equal(got_d, want_d)

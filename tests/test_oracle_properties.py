@@ -1,13 +1,12 @@
-"""Property tests of the oracle (CPU, hypothesis): size-independent invariants of the LPG / silog arithmetic and, when
-/root/reference is mounted, agreement with the unmodified reference modules on randomly drawn shapes (the reference
-ships no tests of its own -- SURVEY 4 -- so shapes beyond the committed golden vectors are pinned this way)."""
+"""Property tests of the oracle (CPU, hypothesis): size-independent invariants of the LPG / silog arithmetic, and
+agreement with the unmodified reference module on randomly drawn shapes, stored in tests/golden/lpg_shapes.npz (the
+reference ships no tests of its own -- SURVEY 4 -- so shapes beyond the other golden vectors are pinned this way)."""
 import numpy as np
 import torch
 from hypothesis import given, settings, strategies as st
 
 import bts_oracle as O
 from conftest import head_planes
-from ref_shim import load_reference, reference_available
 
 shapes = st.tuples(st.integers(1, 3), st.integers(1, 6), st.integers(1, 7), st.sampled_from([2, 4, 8]),
                    st.integers(0, 10 ** 6))
@@ -59,13 +58,9 @@ def test_silog_is_invariant_to_a_common_scale(seed, a):
     assert abs(float(l1) - float(l2)) <= 1e-4 * max(1.0, abs(float(l1)))
 
 
-@settings(max_examples=12, deadline=None)
-@given(shapes)
-def test_lpg_matches_the_live_reference_module_on_random_shapes(s):
-    if not reference_available():
-        return
-    B, h, w, r, seed = s
-    ref = load_reference()
-    plane = head_planes(B, h, w, 10.0, seed=seed)
-    want = ref.local_planar_guidance(r)(plane, torch.full((B,), 518.8579))
-    assert np.array_equal(O.lpg_forward(plane, r).numpy(), want.squeeze(1).numpy() if want.dim() == 4 else want.numpy())
+def test_lpg_matches_the_live_reference_module_on_random_shapes(golden):
+    g = golden("lpg_shapes")
+    assert len(g["cases"]) == 12
+    for j, (B, h, w, r, seed) in enumerate(g["cases"].tolist()):
+        plane = head_planes(B, h, w, 10.0, seed=seed)
+        assert np.array_equal(O.lpg_forward(plane, r).numpy(), g["depth%d" % j]), (B, h, w, r, seed)
