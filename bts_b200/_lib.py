@@ -121,6 +121,7 @@ SIGNATURES = {
     "bts_avgpool2_fwd": [_p, _ll, _i, _i, _i, _i, _p, _ll, _p],
     "bts_avgpool2_bwd": [_p, _ll, _i, _i, _i, _i, _p, _ll, _p],
     "bts_bn_add_relu": [_p, _ll, _ll, _i, _p, _p, _p, _ll, _p, _ll, _p],
+    "bts_bn_add": [_p, _ll, _ll, _i, _p, _p, _p, _ll, _p, _ll, _p],
     "bts_relu_bwd": [_p, _ll, _p, _ll, _ll, _i, _p, _ll, _p],
     "bts_maxpool3s2_fwd": [_p, _ll, _i, _i, _i, _i, _p, _ll, _p, _p],
     "bts_maxpool3s2_bwd": [_p, _ll, _p, _i, _i, _i, _i, _p, _ll, _p],
@@ -136,8 +137,13 @@ SIGNATURES = {
     "bts_conv_pw_fwd_eligible": [_i, _i],
     "bts_conv_pw_fwd": [_p, _ll, _ll, _i, _p, _ll, _ll, _i, _i, _p, _ll, _p],
     "bts_conv_pw_wgrad": [_p, _ll, _p, _ll, _ll, _i, _i, _p, _p, _ll, _ll, _p],
+    "bts_dw_partials": [_i, _i, _i, _i, _i],
+    "bts_dw_fwd": [_p, _ll, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _ll, _p, _p, _p],
+    "bts_dw_dgrad": [_p, _ll, _i, _i, _i, _i, _i, _p, _p, _ll, _p],
+    "bts_dw_wgrad": [_p, _ll, _i, _i, _i, _i, _i, _p, _p, _p, _ll, _p, _p, _ll, _ll, _ll, _p],
 }
-RESTYPES = {"bts_conv_packed_floats": ctypes.c_longlong, "bts_conv_packed_floats_grouped": ctypes.c_longlong, "bts_conv_pw_wgrad_workspace_floats": ctypes.c_longlong}
+RESTYPES = {"bts_conv_packed_floats": ctypes.c_longlong, "bts_conv_packed_floats_grouped": ctypes.c_longlong, "bts_conv_pw_wgrad_workspace_floats": ctypes.c_longlong,
+            "bts_dw_partials": ctypes.c_longlong}
 
 
 def lib():

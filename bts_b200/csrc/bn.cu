@@ -18,9 +18,11 @@ namespace {
 // Column reductions over NHWC: a 256-thread block covers up to 256 channels (64 channel quads) x `rows` pixels; with
 // fewer channels the spare threads take extra pixel rows.  Four independent 16-byte loads per tensor are in flight per
 // thread; the row groups of a block are combined in shared memory, then ONE fp64 atomic per channel per block.
+// `relu`: 0 none, 1 ReLU (mask y > 0); RELU6 (host flag relu == 2) replaces that mask by 0 < y < 6, strict: torch's
+// hardtanh_backward of an in-place ReLU6.  A separate instantiation, so the relu 0 / 1 code is unchanged by it.
 // MODE 0: forward statistics; 1: backward sums; 2: backward sums AND out += [y>0]*scale*g in the same pass (the part of dx
 // that does not depend on the sums -- the k1*x + k0 remainder is deferred, see bts_bn_relu_bwd_fused).
-template <int MODE>
+template <int MODE, bool RELU6 = false>
 __global__ void __launch_bounds__(256) bn_reduce_kernel(const float *__restrict__ x, long long xs, const float *__restrict__ g,
                                                         long long gs, long long M, int C, int rows,
                                                         const float *__restrict__ scale, const float *__restrict__ shift,
@@ -60,7 +62,7 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const float *__restrict_
                     a1[e] = fmaf(xv[e], xv[e], a1[e]);
                 } else {
                     const float y = fmaf(xv[e], sc[e], sh[e]);
-                    const float gm = (!relu || y > 0.f) ? gv[e] : 0.f;
+                    const float gm = (RELU6 ? (y > 0.f && y < 6.f) : (!relu || y > 0.f)) ? gv[e] : 0.f;
                     a0[e] += gm;
                     a1[e] = fmaf(gm, (xv[e] - mu[e]) * is[e], a1[e]);
                     if (ACC) ov[e] = fmaf(sc[e], gm, ov[e]);
@@ -237,7 +239,9 @@ __global__ void bn_fold_kernel(int C, const float *__restrict__ gamma, const flo
     invstd[c] = is;
 }
 
-// dx = [y>0]*scale*g + k1*x + k0  (train; coef = (k0,k1) from bn_bwd_coef_kernel)   or   [y>0]*scale*g  (coef == null)
+// dx = [y>0]*scale*g + k1*x + k0  (train; coef = (k0,k1) from bn_bwd_coef_kernel)   or   [y>0]*scale*g  (coef == null);
+// RELU6: the mask is [0 < y < 6]
+template <bool RELU6>
 __global__ void __launch_bounds__(256) bn_relu_bwd_apply_kernel(const float *__restrict__ x, long long xs,
                                                                 const float *__restrict__ g, long long gs, long long M,
                                                                 int C, const float *__restrict__ scale,
@@ -288,7 +292,7 @@ __global__ void __launch_bounds__(256) bn_relu_bwd_apply_kernel(const float *__r
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
             const float y = fmaf(xv[e], sc[e], sh[e]);
-            float d = (!relu || y > 0.f) ? sc[e] * gv[e] : 0.f;
+            float d = (RELU6 ? (y > 0.f && y < 6.f) : (!relu || y > 0.f)) ? sc[e] * gv[e] : 0.f;
             d += fmaf(xv[e], k1[e], k0[e]);
             r[e] = ov[e] + d;
         }
@@ -382,8 +386,12 @@ extern "C" int bts_bn_bwd_reduce(const float *x, long long x_pixel_stride, const
     const int cg = (C + 255) / 256;
     const int rows = reduce_rows(M, cg);
     dim3 grid((unsigned)((M + rows - 1) / rows), (unsigned)cg);
-    bn_reduce_kernel<1><<<grid, 256, 0, st>>>(x, x_pixel_stride, g, g_pixel_stride, M, C, rows, scale, shift, mean, invstd,
-                                              S1, S2, relu, nullptr, 0);
+    if (relu == 2)
+        bn_reduce_kernel<1, true><<<grid, 256, 0, st>>>(x, x_pixel_stride, g, g_pixel_stride, M, C, rows, scale, shift, mean,
+                                                        invstd, S1, S2, relu, nullptr, 0);
+    else
+        bn_reduce_kernel<1><<<grid, 256, 0, st>>>(x, x_pixel_stride, g, g_pixel_stride, M, C, rows, scale, shift, mean, invstd,
+                                                  S1, S2, relu, nullptr, 0);
     BTS_LAUNCH_CHECK();
     bn_bwd_coef_kernel<<<(C + 127) / 128, 128, 0, st>>>(S1, S2, M, C, scale, mean, invstd, coef);
     BTS_LAUNCH_CHECK();
@@ -458,9 +466,12 @@ extern "C" int bts_bn_bwd_apply(const float *x, long long x_pixel_stride, const 
     long long grid = (total + 255) / 256;
     const long long cap = (long long)bts_num_sms() * 16;
     if (grid > cap) grid = cap;
-    bn_relu_bwd_apply_kernel<<<(int)grid, 256, 0, (cudaStream_t)stream>>>(x, x_pixel_stride, g, g_pixel_stride, M, C, scale,
-                                                                          shift, coef, out, out_pixel_stride, accumulate,
-                                                                          relu);
+    if (relu == 2)
+        bn_relu_bwd_apply_kernel<true><<<(int)grid, 256, 0, (cudaStream_t)stream>>>(
+            x, x_pixel_stride, g, g_pixel_stride, M, C, scale, shift, coef, out, out_pixel_stride, accumulate, relu);
+    else
+        bn_relu_bwd_apply_kernel<false><<<(int)grid, 256, 0, (cudaStream_t)stream>>>(
+            x, x_pixel_stride, g, g_pixel_stride, M, C, scale, shift, coef, out, out_pixel_stride, accumulate, relu);
     BTS_LAUNCH_CHECK();
     return 0;
 }

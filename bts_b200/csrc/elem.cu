@@ -3,7 +3,8 @@
 // sm_100a, HBM-bound.  All tensors are fp32 NHWC with an explicit pixel stride, so a channel slice of a wider slab is
 // read or written in place (concat = one vectorised slice copy per input instead of CatArrayBatchedCopy).
 //
-//   bts_bn_apply       out = x*scale + shift [ReLU]                    BatchNorm apply (train or folded eval stats)
+//   bts_bn_apply       out = x*scale + shift [ReLU | ReLU6]            BatchNorm apply (train or folded eval stats)
+//   bts_bn_add         out = x*scale + shift + res                     MobileNetV2 inverted-residual tail
 //   bts_elu_bwd        out = gy * (y > 0 ? 1 : y + 1)                  ELU'(a) expressed through the saved OUTPUT y
 //   bts_upsample2_sum  out[b,y,x,c] = sum of the 2x2 block of g        backward of the nearest x2 up-sample folded into
 //                      [* (x > 0) when relu_src != null]               upconv's im2col map (+ the ReLU in front of upconv5)
@@ -29,6 +30,8 @@ __host__ inline int stream_grid(long long items) {
 
 __device__ __forceinline__ bool al16(const void *p) { return (((uintptr_t)p) & 15u) == 0; }
 
+// RELU6 (host flag relu == 2): clamp(., 0, 6) instead of the ReLU; a separate instantiation leaves the relu 0 / 1 code as is
+template <bool RELU6>
 __global__ void __launch_bounds__(TPB) bn_apply_kernel(const float *__restrict__ x, long long xs, long long M, int C,
                                                        const float *__restrict__ scale, const float *__restrict__ shift,
                                                        int relu, float *__restrict__ out, long long os) {
@@ -43,12 +46,16 @@ __global__ void __launch_bounds__(TPB) bn_apply_kernel(const float *__restrict__
             const float4 s = __ldg(reinterpret_cast<const float4 *>(scale + c));
             const float4 h = __ldg(reinterpret_cast<const float4 *>(shift + c));
             float4 r = make_float4(fmaf(q.x, s.x, h.x), fmaf(q.y, s.y, h.y), fmaf(q.z, s.z, h.z), fmaf(q.w, s.w, h.w));
-            if (relu) { r.x = fmaxf(r.x, 0.f); r.y = fmaxf(r.y, 0.f); r.z = fmaxf(r.z, 0.f); r.w = fmaxf(r.w, 0.f); }
+            if (RELU6) {
+                r.x = fminf(fmaxf(r.x, 0.f), 6.f); r.y = fminf(fmaxf(r.y, 0.f), 6.f);
+                r.z = fminf(fmaxf(r.z, 0.f), 6.f); r.w = fminf(fmaxf(r.w, 0.f), 6.f);
+            } else if (relu) { r.x = fmaxf(r.x, 0.f); r.y = fmaxf(r.y, 0.f); r.z = fmaxf(r.z, 0.f); r.w = fmaxf(r.w, 0.f); }
             *reinterpret_cast<float4 *>(out + m * os + c) = r;
         } else {
             for (int e = 0; e < 4 && c + e < C; ++e) {
                 float r = fmaf(x[m * xs + c + e], scale[c + e], shift[c + e]);
-                if (relu) r = fmaxf(r, 0.f);
+                if (RELU6) r = fminf(fmaxf(r, 0.f), 6.f);
+                else if (relu) r = fmaxf(r, 0.f);
                 out[m * os + c + e] = r;
             }
         }
@@ -200,7 +207,9 @@ __global__ void __launch_bounds__(TPB) avgpool2_kernel(const float *__restrict__
 }
 
 // ResNet / ResNeXt bottleneck tail (torchvision Bottleneck.forward: out = relu(bn3(conv3) + identity)):
-//   out = max(x*scale + shift + res, 0)
+//   out = max(x*scale + shift + res, 0);   RELU = false: out = x*scale + shift + res (MobileNetV2 InvertedResidual:
+//   x + bn3(conv3), no activation)
+template <bool RELU>
 __global__ void __launch_bounds__(TPB) bn_add_relu_kernel(const float *__restrict__ x, long long xs, long long M, int C,
                                                           const float *__restrict__ scale, const float *__restrict__ shift,
                                                           const float *__restrict__ res, long long rs,
@@ -219,11 +228,13 @@ __global__ void __launch_bounds__(TPB) bn_add_relu_kernel(const float *__restric
             const float4 h = __ldg(reinterpret_cast<const float4 *>(shift + c));
             float4 r = make_float4(fmaf(q.x, s.x, h.x) + r0.x, fmaf(q.y, s.y, h.y) + r0.y, fmaf(q.z, s.z, h.z) + r0.z,
                                    fmaf(q.w, s.w, h.w) + r0.w);
-            r.x = fmaxf(r.x, 0.f); r.y = fmaxf(r.y, 0.f); r.z = fmaxf(r.z, 0.f); r.w = fmaxf(r.w, 0.f);
+            if (RELU) { r.x = fmaxf(r.x, 0.f); r.y = fmaxf(r.y, 0.f); r.z = fmaxf(r.z, 0.f); r.w = fmaxf(r.w, 0.f); }
             *reinterpret_cast<float4 *>(out + m * os + c) = r;
         } else {
-            for (int e = 0; e < 4 && c + e < C; ++e)
-                out[m * os + c + e] = fmaxf(fmaf(x[m * xs + c + e], scale[c + e], shift[c + e]) + res[m * rs + c + e], 0.f);
+            for (int e = 0; e < 4 && c + e < C; ++e) {
+                const float r = fmaf(x[m * xs + c + e], scale[c + e], shift[c + e]) + res[m * rs + c + e];
+                out[m * os + c + e] = RELU ? fmaxf(r, 0.f) : r;
+            }
         }
     }
 }
@@ -314,8 +325,12 @@ __global__ void __launch_bounds__(TPB) maxpool3s2_bwd_kernel(const float *__rest
 extern "C" int bts_bn_apply(const float *x, long long x_pixel_stride, long long M, int C, const float *scale,
                             const float *shift, int relu, float *out, long long out_pixel_stride, void *stream) {
     if (!x || !scale || !shift || !out || M < 1 || C < 1) return BTS_EINVAL;
-    bn_apply_kernel<<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(x, x_pixel_stride, M, C, scale, shift,
-                                                                                       relu, out, out_pixel_stride);
+    if (relu == 2)
+        bn_apply_kernel<true><<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(x, x_pixel_stride, M, C, scale,
+                                                                                             shift, relu, out, out_pixel_stride);
+    else
+        bn_apply_kernel<false><<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(x, x_pixel_stride, M, C, scale,
+                                                                                              shift, relu, out, out_pixel_stride);
     BTS_LAUNCH_CHECK();
     return 0;
 }
@@ -376,8 +391,17 @@ extern "C" int bts_bn_add_relu(const float *x, long long x_pixel_stride, long lo
                                const float *shift, const float *res, long long res_pixel_stride, float *out,
                                long long out_pixel_stride, void *stream) {
     if (!x || !scale || !shift || !res || !out || M < 1 || C < 1) return BTS_EINVAL;
-    bn_add_relu_kernel<<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(x, x_pixel_stride, M, C, scale, shift, res,
-                                                                                          res_pixel_stride, out, out_pixel_stride);
+    bn_add_relu_kernel<true><<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(
+        x, x_pixel_stride, M, C, scale, shift, res, res_pixel_stride, out, out_pixel_stride);
+    BTS_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int bts_bn_add(const float *x, long long x_pixel_stride, long long M, int C, const float *scale, const float *shift,
+                          const float *res, long long res_pixel_stride, float *out, long long out_pixel_stride, void *stream) {
+    if (!x || !scale || !shift || !res || !out || M < 1 || C < 1) return BTS_EINVAL;
+    bn_add_relu_kernel<false><<<stream_grid(M * ((C + 3) / 4)), TPB, 0, (cudaStream_t)stream>>>(
+        x, x_pixel_stride, M, C, scale, shift, res, res_pixel_stride, out, out_pixel_stride);
     BTS_LAUNCH_CHECK();
     return 0;
 }

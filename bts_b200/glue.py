@@ -9,6 +9,10 @@ run as one of the streaming NHWC kernels of csrc/elem.cu / csrc/bn.cu:
   bn_relu_conv   y = conv(ReLU(BN(x)))                     atrous_conv halves (:51-66), DenseNet transitions
   cat_nhwc       channel concat into a 16-byte-aligned slab (the nine torch.cat of bts.forward); backward = views
   avgpool2       2x2 average pool of the transitions
+  dwconv         depthwise 3x3 conv (padding 1, stride 1 / 2) on csrc/dwconv.cu, forward / dgrad / wgrad
+  bn_add         y = BN(x) + res                           MobileNetV2 inverted-residual tail
+  inverted_residual  torchvision InvertedResidual as ONE unit: expand 1x1 -> BN+ReLU6 folded into the depthwise conv's
+                 prologue -> depthwise 3x3 (BN statistics in its epilogue) -> BN+ReLU6 -> project 1x1 -> BN [+ x]
 
 Each unit is a torch.autograd.Function whose backward launches our kernels too (ELU', BN reductions, wgrad / dgrad on
 the engine, 2x2 gradient fold of the up-sample).  Parameters stay the nn.Modules' own, BatchNorm running statistics are
@@ -161,6 +165,20 @@ def conv_act(x, weight, padding=0, dilation=1, pre_relu=False, up=False, act=Non
 
 
 # ------------------------------------------------------------------------------------------------ BatchNorm (+ ReLU)
+_ACT_CODE = {None: 0, "relu": 1, "relu6": 2}      # the `relu` flag of bts_bn_apply / bts_bn_bwd_reduce / bts_bn_bwd_apply
+
+
+def bn_apply(x, st, relu):
+    """x*scale + shift [ReLU | ReLU6] with (scale, shift) = st[0], st[1]"""
+    x, xs = _nhwc(x)
+    B, C, H, W = x.shape
+    y = _new(B, C, H, W, x.device)
+    _lib.check(_lib.lib().bts_bn_apply(_ptr(x), xs, B * H * W, C, _ptr(st[0]), _ptr(st[1]), int(relu), _ptr(y), C, _stream()),
+               "bts_bn_apply")
+    _lib.count()
+    return y
+
+
 class _BnAct(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, gamma, beta, bn, relu):
@@ -186,10 +204,13 @@ class _BnAct(torch.autograd.Function):
                 S[0].float() if ctx.needs_input_grad[2] else None, None, None)
 
 
-def bn_act(x, bn, relu=False):
+def bn_act(x, bn, relu=False, act=None):
     """nn.BatchNorm2d `bn` applied to x (batch statistics + running-stat update in train mode, folded running
-    statistics in eval mode), optionally followed by ReLU -- 3 streaming kernels forward, 3 backward"""
-    return _BnAct.apply(x, bn.weight, bn.bias, bn, bool(relu))
+    statistics in eval mode), optionally followed by ReLU (relu=True or act="relu") or ReLU6 (act="relu6") -- 3 streaming
+    kernels forward, 3 backward"""
+    if act not in _ACT_CODE:
+        raise ValueError("bn_act: act must be one of %s" % sorted(k for k in _ACT_CODE if k))
+    return _BnAct.apply(x, bn.weight, bn.bias, bn, _ACT_CODE[act] or int(bool(relu)))
 
 
 # ------------------------------------------------------------------------------------------------ BN -> ReLU -> conv
@@ -355,3 +376,208 @@ class _BnAddRelu(torch.autograd.Function):
 def bn_add_relu(x, res, bn):
     """relu(bn(x) + res): the tail of a torchvision Bottleneck, one streaming kernel after the statistics"""
     return _BnAddRelu.apply(x, res, bn.weight, bn.bias, bn)
+
+
+class _BnAdd(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, res, gamma, beta, bn):
+        x, xs = _nhwc(x)
+        res, rs = _nhwc(res)
+        B, C, H, W = x.shape
+        n = B * H * W
+        batch = bn_uses_batch_stats(bn)
+        st = bn_finalize(bn_stats(x) if batch else None, n, bn, gamma, beta, batch)
+        y = _new(B, C, H, W, x.device)
+        _lib.check(_lib.lib().bts_bn_add(_ptr(x), xs, n, C, _ptr(st[0]), _ptr(st[1]), _ptr(res), rs, _ptr(y), C, _stream()),
+                   "bts_bn_add")
+        _lib.count()
+        ctx.batch = batch
+        ctx.save_for_backward(x, st)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, st = ctx.saved_tensors
+        gx, S = bn_backward(x, gy, st, ctx.batch, 0)
+        return (gx if ctx.needs_input_grad[0] else None, gy if ctx.needs_input_grad[1] else None,
+                S[1].float() if ctx.needs_input_grad[2] else None, S[0].float() if ctx.needs_input_grad[3] else None, None)
+
+
+def bn_add(x, res, bn):
+    """bn(x) + res: the tail of a MobileNetV2 inverted residual with its identity connection"""
+    return _BnAdd.apply(x, res, bn.weight, bn.bias, bn)
+
+
+# ------------------------------------------------------------------------------------------------ depthwise 3x3
+def dw_eligible(conv_module):
+    """a depthwise 3x3 / padding 1 / stride 1 or 2 nn.Conv2d without bias that csrc/dwconv.cu computes"""
+    m = conv_module
+    C = m.in_channels
+    return (m.groups == C and m.out_channels == C and C % 4 == 0 and tuple(m.kernel_size) == (3, 3)
+            and tuple(m.padding) == (1, 1) and tuple(m.dilation) == (1, 1) and m.stride[0] == m.stride[1]
+            and m.stride[0] in (1, 2) and m.bias is None and m.padding_mode == "zeros")
+
+
+def _dw_out(H, W, stride):
+    return (H - 1) // stride + 1, (W - 1) // stride + 1
+
+
+def dw_fwd(x, weight, stride, pre=None, post=None, stats=False):
+    """depthwise 3x3 forward: (y, sums).  pre = [4,C] BN state -> input prologue clamp(x*st[0] + st[1], 0, 6);
+    post = [4,C] eval BN state -> epilogue clamp(y*st[0] + st[1], 0, 6); stats -> sums = fp64 [2,C] (sum y, sum y^2)"""
+    x, xs = _nhwc(x)
+    B, C, H, W = x.shape
+    Ho, Wo = _dw_out(H, W, stride)
+    L = _lib.lib()
+    y = _new(B, C, Ho, Wo, x.device)
+    part = sums = None
+    if stats:
+        part = torch.empty(L.bts_dw_partials(B, Ho, Wo, C, 0), device=x.device, dtype=torch.float64)
+        sums = torch.empty((2, C), device=x.device, dtype=torch.float64)
+    w = weight.detach().contiguous()
+    _lib.check(L.bts_dw_fwd(_ptr(x), xs, B, H, W, C, int(stride), _ptr(w),
+                            _ptr(pre[0]) if pre is not None else None, _ptr(pre[1]) if pre is not None else None,
+                            _ptr(post[0]) if post is not None else None, _ptr(post[1]) if post is not None else None,
+                            _ptr(y), C, _ptr(part), _ptr(sums), _stream()), "bts_dw_fwd")
+    _lib.count(2 if stats else 1)
+    return y, sums
+
+
+def dw_dgrad(g, weight, stride, H, W):
+    """d/dx of the depthwise 3x3 conv (input H x W) given g = d/dy"""
+    g, gs = _nhwc(g)
+    B, C = g.shape[0], g.shape[1]
+    gx = _new(B, C, H, W, g.device)
+    w = weight.detach().contiguous()
+    _lib.check(_lib.lib().bts_dw_dgrad(_ptr(g), gs, B, H, W, C, int(stride), _ptr(w), _ptr(gx), C, _stream()),
+               "bts_dw_dgrad")
+    _lib.count()
+    return gx
+
+
+def dw_wgrad(x, g, weight, stride, pre=None):
+    """dW (shaped / strided like the weight) of the depthwise 3x3 conv, the input prologue `pre` recomputed from x"""
+    x, xs = _nhwc(x)
+    g, gs = _nhwc(g)
+    B, C, H, W = x.shape
+    L = _lib.lib()
+    part = torch.empty(L.bts_dw_partials(B, g.shape[2], g.shape[3], C, 1), device=x.device, dtype=torch.float64)
+    gw = torch.empty_strided(tuple(weight.shape), tuple(weight.stride()), device=x.device, dtype=torch.float32)
+    s = weight.stride()
+    _lib.check(L.bts_dw_wgrad(_ptr(x), xs, B, H, W, C, int(stride), _ptr(pre[0]) if pre is not None else None,
+                              _ptr(pre[1]) if pre is not None else None, _ptr(g), gs, _ptr(part), _ptr(gw), s[0], s[2], s[3],
+                              _stream()), "bts_dw_wgrad")
+    _lib.count(2)
+    return gw
+
+
+class _DwConv(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, stride):
+        y, _ = dw_fwd(x, weight, stride)
+        ctx.stride = stride
+        ctx.save_for_backward(x, weight)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, weight = ctx.saved_tensors
+        gx = dw_dgrad(gy, weight, ctx.stride, x.shape[2], x.shape[3]) if ctx.needs_input_grad[0] else None
+        gw = dw_wgrad(x, gy, weight, ctx.stride) if ctx.needs_input_grad[1] else None
+        return gx, gw, None
+
+
+def dwconv(x, weight, stride=1):
+    """depthwise 3x3 conv, padding 1, weight (C,1,3,3): forward, dgrad and wgrad on csrc/dwconv.cu"""
+    return _DwConv.apply(x, weight, int(stride))
+
+
+# ------------------------------------------------------------------------------------------------ MobileNetV2 block
+def _zeros2(C, dev):
+    return torch.zeros((2, C), device=dev, dtype=torch.float64)
+
+
+class _InvertedResidual(torch.autograd.Function):
+    """torchvision InvertedResidual [(1x1 -> BN1 -> ReLU6) -> dw 3x3 -> BN2 -> ReLU6 -> 1x1 -> BN3 (+ x)].  BN1 + ReLU6 run
+    inside the depthwise conv's prologue (the expanded activation is never written), the depthwise conv's epilogue reduces
+    BN2's batch statistics (or, in eval mode without autograd, applies BN2 + ReLU6), the 1x1 convs run on the tcgen05
+    engine.  Saved for backward: x, the raw expand output e, the raw dw output d, the project conv's input a and its
+    output p -- BN1 / BN2 activations are recomputed from e / d."""
+
+    @staticmethod
+    def forward(ctx, x, w1, g1, b1, wdw, g2, b2, w3, g3, b3, bns, stride, residual):
+        bn1, bn2, bn3 = bns
+        x, xs = _nhwc(x)
+        B, _, H, W = x.shape
+        dev = x.device
+        grad = any(ctx.needs_input_grad)
+        t1 = t2 = None
+        st1 = e = None
+        if w1 is not None:
+            t1 = bn_uses_batch_stats(bn1)
+            s1 = _zeros2(w1.shape[0], dev) if t1 and w1.shape[0] <= 256 else None      # stats in the engine epilogue
+            e = conv.conv2d_tc(x, w1, stats=s1)
+            st1 = bn_finalize((s1 if s1 is not None else bn_stats(e)) if t1 else None, B * H * W, bn1, g1, b1, t1)
+        src = e if e is not None else x
+        Ho, Wo = _dw_out(H, W, stride)
+        t2 = bn_uses_batch_stats(bn2)
+        d = None
+        if not t2 and not grad:          # eval without autograd: BN2 + ReLU6 in the depthwise epilogue
+            st2 = bn_finalize(None, B * Ho * Wo, bn2, g2, b2, False)
+            a, _ = dw_fwd(src, wdw, stride, pre=st1, post=st2)
+        else:
+            d, s2 = dw_fwd(src, wdw, stride, pre=st1, stats=t2)
+            st2 = bn_finalize(s2, B * Ho * Wo, bn2, g2, b2, t2)
+            a = bn_apply(d, st2, 2)
+        t3 = bn_uses_batch_stats(bn3)
+        Co = w3.shape[0]
+        s3 = _zeros2(Co, dev) if t3 and Co <= 256 else None
+        p = conv.conv2d_tc(a, w3, stats=s3)
+        st3 = bn_finalize((s3 if s3 is not None else bn_stats(p)) if t3 else None, B * Ho * Wo, bn3, g3, b3, t3)
+        y = _new(B, Co, Ho, Wo, dev)
+        L = _lib.lib()
+        if residual:
+            _lib.check(L.bts_bn_add(_ptr(p), Co, B * Ho * Wo, Co, _ptr(st3[0]), _ptr(st3[1]), _ptr(x), xs, _ptr(y), Co,
+                                    _stream()), "bts_bn_add")
+        else:
+            _lib.check(L.bts_bn_apply(_ptr(p), Co, B * Ho * Wo, Co, _ptr(st3[0]), _ptr(st3[1]), 0, _ptr(y), Co, _stream()),
+                       "bts_bn_apply")
+        _lib.count()
+        if grad:
+            ctx.cfg = (stride, residual, t1, t2, t3)
+            ctx.save_for_backward(x, e, d, a, p, st1, st2, st3, w1, wdw, w3)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, e, d, a, p, st1, st2, st3, w1, wdw, w3 = ctx.saved_tensors
+        stride, residual, t1, t2, t3 = ctx.cfg
+        need = ctx.needs_input_grad
+        gy, _ = _nhwc(gy)
+        gp, S3 = bn_backward(p, gy, st3, t3, 0)
+        gw3 = conv.wgrad_tc(a, gp, w3.shape, w3.stride()) if need[7] else None
+        ga = conv.conv2d_tc(gp, w3, 1, 0, 1, transpose_flip=True)
+        gd, S2 = bn_backward(d, ga, st2, t2, 2, out=ga)                    # in place on the dgrad result
+        src = e if e is not None else x
+        gwdw = dw_wgrad(src, gd, wdw, stride, pre=st1) if need[4] else None
+        gx = gw1 = S1 = None
+        if e is not None:
+            ge, S1 = bn_backward(e, dw_dgrad(gd, wdw, stride, e.shape[2], e.shape[3]), st1, t1, 2)
+            gw1 = conv.wgrad_tc(x, ge, w1.shape, w1.stride()) if need[1] else None
+            if need[0]:
+                gx = conv.conv2d_tc(ge, w1, 1, 0, 1, transpose_flip=True)
+        elif need[0]:
+            gx = dw_dgrad(gd, wdw, stride, x.shape[2], x.shape[3])
+        if gx is not None and residual:
+            copy_channels(gy, gx, accumulate=True)
+        f = lambda S, i, k: S[k].float() if (S is not None and need[i]) else None
+        return (gx, gw1, f(S1, 2, 1), f(S1, 3, 0), gwdw, f(S2, 5, 1), f(S2, 6, 0), gw3, f(S3, 8, 1), f(S3, 9, 0),
+                None, None, None)
+
+
+def inverted_residual(x, expand, bn1, dw, bn2, project, bn3, residual):
+    """torchvision InvertedResidual forward on our kernels; `expand` / `bn1` are None for the t = 1 block"""
+    return _InvertedResidual.apply(x, expand.weight if expand is not None else None,
+                                   bn1.weight if bn1 is not None else None, bn1.bias if bn1 is not None else None,
+                                   dw.weight, bn2.weight, bn2.bias, project.weight, bn3.weight, bn3.bias, (bn1, bn2, bn3),
+                                   int(dw.stride[0]), bool(residual))

@@ -68,6 +68,10 @@ class Conv2dTC(nn.Conv2d):
                     return conv.conv_c1(x, self.weight, sigmoid=False)
                 return conv.conv2d(x, self.weight, self.stride[0], self.padding[0], self.dilation[0])
             cpg = self.in_channels // self.groups
+            from . import glue
+            if glue.dw_eligible(self):
+                # depthwise 3x3 (MobileNetV2): CUDA-core streaming kernels, fwd / dgrad / wgrad
+                return glue.dwconv(x, self.weight, self.stride[0])
             if (self.in_channels == self.out_channels and cpg >= 4 and conv.group_window(self.out_channels, cpg) == 128):
                 # ResNeXt grouped 3x3 (32 groups): block-diagonal operator on the engine, fwd / dgrad / wgrad
                 return conv.conv2d(x, self.weight, self.stride[0], self.padding[0], self.dilation[0], groups=self.groups)
@@ -174,16 +178,74 @@ def _dense_block_class():
     return _DenseBlock, DenseBlockTC
 
 
+def _mobilenet_classes():
+    from torchvision.models.mobilenetv2 import InvertedResidual
+    from torchvision.ops.misc import Conv2dNormActivation
+
+    def conv_bn_relu6(seq):
+        """(conv, bn) of a Conv2dNormActivation [Conv2d(no bias), affine BatchNorm2d, ReLU6], else None"""
+        if len(seq) == 3 and isinstance(seq[0], nn.Conv2d) and seq[0].bias is None and type(seq[1]) is nn.BatchNorm2d \
+                and seq[1].affine and isinstance(seq[2], nn.ReLU6):
+            return seq[0], seq[1]
+        return None
+
+    class ConvBnReLU6TC(Conv2dNormActivation):
+        """torchvision Conv2dNormActivation [conv -> BN -> ReLU6] (the MobileNetV2 stem and last 1x1 layer): the conv on the
+        engine (or the depthwise kernels), BN + ReLU6 on our streaming kernels; parameters / buffers / state_dict untouched"""
+
+        def forward(self, x):
+            parts = conv_bn_relu6(self)
+            if not (fuse_enabled(x) and parts):
+                return super().forward(x)
+            from . import glue
+            return glue.bn_act(parts[0](x), parts[1], act="relu6")
+
+    class InvertedResidualTC(InvertedResidual):
+        """torchvision MobileNetV2 block [(1x1 -> BN -> ReLU6) -> dw 3x3 -> BN -> ReLU6 -> 1x1 -> BN (+ x)] as one fused
+        autograd unit (glue.inverted_residual); parameters / buffers / state_dict untouched"""
+
+        def _parts(self):
+            layers = list(self.conv)
+            if len(layers) not in (3, 4):
+                return None
+            expand = conv_bn_relu6(layers[0]) if len(layers) == 4 else (None, None)
+            dw = conv_bn_relu6(layers[-3])
+            project, bn3 = layers[-2], layers[-1]
+            if expand is None or dw is None or not (isinstance(project, nn.Conv2d) and project.bias is None
+                                                   and tuple(project.kernel_size) == (1, 1) and project.stride == (1, 1)
+                                                   and type(bn3) is nn.BatchNorm2d and bn3.affine):
+                return None
+            if expand[0] is not None and (tuple(expand[0].kernel_size) != (1, 1) or expand[0].stride != (1, 1)
+                                          or expand[0].groups != 1):
+                return None
+            return expand[0], expand[1], dw[0], dw[1], project, bn3
+
+        def forward(self, x):
+            from . import glue
+            parts = self._parts()
+            if not (fuse_enabled(x) and parts and glue.dw_eligible(parts[2])):
+                return super().forward(x)
+            return glue.inverted_residual(x, *parts, residual=self.use_res_connect)
+
+    return InvertedResidual, InvertedResidualTC, Conv2dNormActivation, ConvBnReLU6TC
+
+
 def adopt_convs(module):
-    """Re-class every eligible nn.Conv2d (-> Conv2dTC) and DenseNet block (-> fused DenseBlockTC) of a torchvision
-    module tree in place -- parameter names, shapes and init are untouched."""
+    """Re-class every eligible nn.Conv2d (-> Conv2dTC), DenseNet block (-> fused DenseBlockTC), ResNet bottleneck and
+    MobileNetV2 block / conv-BN-ReLU6 layer of a torchvision module tree in place -- parameter names, shapes and init are
+    untouched."""
     base, fusedcls = _dense_block_class()
     tbase, tcls = _transition_class()
     bbase, bcls = _bottleneck_class()
+    ibase, icls, cbase, ccls = _mobilenet_classes()
     resnet = any(type(m) is bbase for m in module.modules())
     for m in module.modules():
         if type(m) is nn.Conv2d:
             m.__class__ = Conv2dTC
+        elif type(m) is ibase:
+            m.__class__ = icls
+        elif type(m) is cbase:
+            m.__class__ = ccls
         elif type(m) is base:
             m.__class__ = fusedcls
         elif type(m) is tbase:

@@ -232,7 +232,8 @@ int bts_bn_relu_bwd_apply(const float *x, long long x_pixel_stride, const float 
                           long long out_pixel_stride, int accumulate, void *stream);
 
 /* generalised forms with an explicit `relu` flag (relu=0: plain BatchNorm, as the decoder's bn5/bn4/bn4_2/bn3/bn2 which
- * feed a concat, bts.py:200-246); the *_relu_* entry points above are these with relu=1. */
+ * feed a concat, bts.py:200-246; relu=2: ReLU6, mask 0 < y < 6 strictly, the MobileNetV2 BN + ReLU6); the *_relu_* entry
+ * points above are these with relu=1. */
 int bts_bn_bwd_reduce(const float *x, long long x_pixel_stride, const float *g, long long g_pixel_stride, long long M,
                       int C, const float *scale, const float *shift, const float *mean, const float *invstd, int relu,
                       double *S1, double *S2, float *coef, void *stream);
@@ -254,7 +255,8 @@ int bts_bn_bwd_correct(const float *x, long long x_pixel_stride, long long M, in
 /* ---- streaming NHWC glue kernels of the decoder / encoder transitions (csrc/elem.cu) ---------------------------
  * All take explicit pixel strides (floats) so channel slices of wider slabs are read / written in place.
  *   bts_bn_apply       out = x*scale + shift [, ReLU]   -- BatchNorm2d forward given (scale, shift) from bts_bn_finalize /
- *                      bts_bn_fold (decoder BNs bts.py:154-182; torchvision norm0 / norm5)
+ *                      bts_bn_fold (decoder BNs bts.py:154-182; torchvision norm0 / norm5); relu: 0 none, 1 ReLU,
+ *                      2 ReLU6 = clamp(., 0, 6) (MobileNetV2 Conv2dNormActivation)
  *   bts_elu_bwd        out = gy * (y > 0 ? 1 : y + 1)   -- backward of nn.ELU() through its saved OUTPUT y (bts.py:72,79,...)
  *   bts_upsample2_sum  out[b,y,x,:] = sum of g[b,2y..2y+1,2x..2x+1,:]  -- backward of F.interpolate(scale_factor=2,
  *                      mode='nearest') (bts.py:77); relu_src != NULL additionally gates by relu_src > 0 (torch.nn.ReLU in
@@ -297,12 +299,37 @@ int bts_conv_pw_wgrad(const float *x, long long x_pixel_stride, const float *dy,
  *                     winning window position (uint8 per OUTPUT element, dense [B,Ho,Wo,C]) -> deterministic gather backward */
 int bts_bn_add_relu(const float *x, long long x_pixel_stride, long long M, int C, const float *scale, const float *shift,
                     const float *res, long long res_pixel_stride, float *out, long long out_pixel_stride, void *stream);
+/*   bts_bn_add        out = x*scale + shift + res                    MobileNetV2 InvertedResidual tail  x + bn3(conv3(.)) */
+int bts_bn_add(const float *x, long long x_pixel_stride, long long M, int C, const float *scale, const float *shift,
+               const float *res, long long res_pixel_stride, float *out, long long out_pixel_stride, void *stream);
 int bts_relu_bwd(const float *gy, long long gy_pixel_stride, const float *y, long long y_pixel_stride, long long M, int C,
                  float *out, long long out_pixel_stride, void *stream);
 int bts_maxpool3s2_fwd(const float *x, long long x_pixel_stride, int B, int H, int W, int C, float *out,
                        long long out_pixel_stride, unsigned char *argmax, void *stream);
 int bts_maxpool3s2_bwd(const float *g, long long g_pixel_stride, const unsigned char *argmax, int B, int H, int W, int C,
                        float *gx, long long gx_pixel_stride, void *stream);
+
+/* ---- depthwise 3x3 convolution, padding 1, stride 1 or 2, of the MobileNetV2 inverted residuals (torchvision
+ * mobilenetv2.py behind reference pytorch/bts.py:298-300), csrc/dwconv.cu.  fp32 NHWC with explicit pixel strides
+ * (multiples of 4, 16-byte aligned bases), C % 4 == 0; w = the contiguous (C,1,3,3) weight, read on every call.
+ * Hout = (H-1)/stride + 1, likewise Wout.
+ *   bts_dw_fwd   y = dw(act_in(x)); act_in(x) = clamp(x*pre_scale + pre_shift, 0, 6) when pre_* != NULL, else x
+ *                (out-of-bounds taps are 0 after the activation).  Epilogue: sums != NULL -> sums[0][c] = sum y,
+ *                sums[1][c] = sum y^2 (fp64 [2][C], deterministic two-pass reduction through `partials`);
+ *                post_* != NULL -> y = clamp(y*post_scale + post_shift, 0, 6) (a folded eval-mode BN + ReLU6).
+ *   bts_dw_dgrad gx (B,H,W,C) = d/dx of the plain depthwise conv given g (B,Hout,Wout,C); gather form, no atomics.
+ *   bts_dw_wgrad dw[c*s_c + ky*s_kh + kx*s_kw] = sum_p g[p,c] * act_in(x)[p*stride + (ky-1, kx-1), c]; deterministic
+ *                two-pass reduction through `partials`.
+ * partials: bts_dw_partials(B, Hout, Wout, C, wgrad) doubles (wgrad = 0 for the forward statistics, 1 for bts_dw_wgrad). */
+long long bts_dw_partials(int B, int Hout, int Wout, int C, int wgrad);
+int bts_dw_fwd(const float *x, long long x_pixel_stride, int B, int H, int W, int C, int stride, const float *w,
+               const float *pre_scale, const float *pre_shift, const float *post_scale, const float *post_shift, float *y,
+               long long y_pixel_stride, double *partials, double *sums, void *stream);
+int bts_dw_dgrad(const float *g, long long g_pixel_stride, int B, int H, int W, int C, int stride, const float *w, float *gx,
+                 long long gx_pixel_stride, void *stream);
+int bts_dw_wgrad(const float *x, long long x_pixel_stride, int B, int H, int W, int C, int stride, const float *pre_scale,
+                 const float *pre_shift, const float *g, long long g_pixel_stride, double *partials, float *dw, long long s_c,
+                 long long s_kh, long long s_kw, void *stream);
 
 /* ---- optimizer step of the training loop (reference pytorch/bts_main.py:371-373 torch.optim.AdamW, two groups, eps 1e-3;
  * :456-460 poly LR) as ONE multi-tensor kernel, csrc/optim.cu.  ptrs: device int64 [4n] = param | grad | exp_avg | exp_avg_sq
